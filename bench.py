@@ -474,6 +474,31 @@ def load_synth_(module, dev, seed: int) -> None:
 
 
 PARITY_TOL = {"rel_l2": 3e-2, "cosine": 0.999}   # DESIGN.md section 4 (bf16 path vs the fp32 reference)
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, arrays: dict, limit_bytes: int = DUMP_LIMIT_BYTES) -> dict:
+    """Write each array as out_dir/<name>.npy in float32, so that two builds can be compared output for output.
+    When the arrays together would exceed `limit_bytes`, each is replaced by the same share of its elements: a flat
+    sample at indices drawn with a fixed seed and sorted (identical from run to run for the same shapes).
+    -> {name: {"shape", "dtype", "sampled_elements" (None: complete)}}"""
+    import numpy as np
+
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.size for a in arrays.values())
+    keep = (limit_bytes - 128 * len(arrays)) // 4     # each .npy header takes 128 bytes
+    info = {}
+    for name, a in arrays.items():
+        sampled = None
+        flat = a.reshape(-1)
+        if total > keep:
+            sampled = a.size * keep // total
+            flat = flat[np.sort(np.random.default_rng(0).choice(a.size, sampled, replace=False))]
+        np.save(out_dir / f"{name}.npy", flat if sampled is not None else a)
+        info[name] = {"shape": list(a.shape), "dtype": "float32", "sampled_elements": sampled}
+    return info
 
 
 def parity_check(eng, dev, manifest) -> dict:
@@ -503,16 +528,22 @@ def parity_check(eng, dev, manifest) -> dict:
     with torch.no_grad():
         out = eng.model.diffusion_model(xin, gold["timesteps"].to(dev), ctx, y, None, T,
                                         torch.zeros(2, T, device=dev))
-    res = {"unet_forward": {"rel_l2": rel(out, gold["out"]), "cosine": cos(out, gold["out"]),
+    st = gold["stride"]
+    res = {"unet_forward": {"rel_l2": rel(out[:, :, ::st, ::st], gold["out_sub"]),
+                            "cosine": cos(out[:, :, ::st, ::st], gold["out_sub"]),
+                            "rel_l2_full_items": rel(out[gold["full_items"]], gold["out_full"]),
                             "finite": bool(torch.isfinite(out).all()), "fixture": "tests/golden/unet_v3d512.pt"}}
     md = manifest["decoder_v3d512"]
     gold = torch.load(gold_dir / "decoder_v3d512.pt")
+    z = synth.synth_latents(md["B"], md["latent_hw"], seed=md["z_seed"])
+    if not torch.equal(z[:, :, ::16, ::16], gold["z_check"]):
+        raise SystemExit("bench.py: the decoder fixture's latents do not regenerate from their seed")
     with torch.no_grad():
-        img = eng.first_stage_model.decoder(gold["z"].to(dev) / 0.18215, timesteps=md["T"])
-    st = gold["stride"]
+        img = eng.first_stage_model.decoder(z.to(dev) / 0.18215, timesteps=md["T"])
+    st, crop = gold["stride"], gold["crop"]
     res["decode"] = {"rel_l2": rel(img[:, :, ::st, ::st], gold["out_sub"]),
                      "cosine": cos(img[:, :, ::st, ::st], gold["out_sub"]),
-                     "rel_l2_full_frames": rel(img[gold["full_frames"]], gold["out_full"]),
+                     "rel_l2_full_frames": rel(img[gold["full_frames"], :, :crop, :crop], gold["out_full"]),
                      "finite": bool(torch.isfinite(img).all()), "fixture": "tests/golden/decoder_v3d512.pt"}
     res["tolerance"] = dict(PARITY_TOL)
     res["against"] = "outputs of the real reference modules (fp32, CPU) on the same seeded weights and inputs"
@@ -764,14 +795,15 @@ def run_native(args) -> None:
         l0 = ops.launch_count() + eng.model.diffusion_model.replayed_launches
         w0 = time.time()
         ev0.record()
-        for _ in range(k):
+        for _ in range(k - 1):
             fn()
+        out = fn()      # kept for --dump-outputs; earlier results are dropped at once, as the caching allocator expects
         ev1.record()
         torch.cuda.synchronize()
         w1 = time.time()
         parallel.barrier()
         secs = parallel.max_over_ranks(ev0.elapsed_time(ev1) / 1000.0, dev)
-        return secs, ops.launch_count() + eng.model.diffusion_model.replayed_launches - l0, (w0, w1)
+        return secs, ops.launch_count() + eng.model.diffusion_model.replayed_launches - l0, (w0, w1), out
 
     for _ in range(args.warmup):
         step_resident()
@@ -781,11 +813,16 @@ def run_native(args) -> None:
     if rank == 0:
         clocks.start()
         time.sleep(0.3)
-    secs, launches, (w0, w1) = timed(step_resident, args.steps)
+    secs, launches, (w0, w1), frames = timed(step_resident, args.steps)
     clk = clocks.stop(w0, w1) if rank == 0 else None
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # the uint8 THWC frames the hot path returned in the last timed step (rank 0's image or frame block)
+        dumped = dump_outputs(args.dump_outputs, {"frames": frames.cpu().numpy()})
+    del frames
 
     step_e2e()  # warm the e2e-only pieces (pinned copies)
-    secs_e2e, _, _ = timed(step_e2e, args.steps)
+    secs_e2e, _, _, _ = timed(step_e2e, args.steps)
 
     # ---- roofline of the dominant kernel family + per-family breakdown: every launch of ONE step is bracketed
     #      by CUDA events on the launching stream (a separate pass, so the timed region above carries no probes)
@@ -886,6 +923,8 @@ def run_native(args) -> None:
         decode_families={k: [ms(a, b) for a, b in v] for k, v in decode_families.items()},
         decode_shapes={k: [(f, ms(a, b)) for f, a, b in v] for k, v in decode_shapes.items()})
     line["parity"] = parity
+    if dumped is not None:
+        line["dumped_outputs"] = dumped
     if plan is not None:
         line["exchanges_ms_per_step"] = summarise_exchanges(xchg_events, ms(pe0, pe1))
     elif world > 1 and not args.no_strong:
@@ -927,7 +966,14 @@ def main():
                     help="images (default): one image per GPU, weak scaling.  ONE image over the GPUs (strong scaling): "
                          "views = frame blocks (K|V all-gather, conv halos, 3-D GroupNorm all-reduce); cfg = the [uc; c] "
                          "halves on 2 GPUs (one all-gather per network evaluation); cfg+views = both (>= 4 GPUs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned in its last step (the uint8 frames "
+                         "[T, H, W, 3] of rank 0) as DIR/frames.npy in float32; a fixed seeded sample when over 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs needs the native arm: the reference arm times pieces of the path, not the path")
     if args.warmup < 3 and args.impl == "native":
         print("warning: timing rules ask for >= 3 warm-up steps", file=sys.stderr)
     if args.impl == "reference":

@@ -10,6 +10,7 @@ unless they agree to <= 2e-4 of the output scale.  Only the reference's outputs 
 """
 from __future__ import annotations
 
+import gzip
 import importlib
 import json
 import sys
@@ -34,7 +35,7 @@ def _pin(name: str, ref: torch.Tensor, ora: torch.Tensor) -> float:
 
 
 def _unet_case(ns, tag: str, model_channels: int, T: int, hw: int, wseed: int, sigma: float, manifest: dict,
-               tap_stride: int = 1):
+               tap_stride: int = 1, full_items=None, stride: int = 1):
     kw = dict(reference_shim.V3D_UNET_KW)
     kw["model_channels"] = model_channels
     net = ns.video_model.VideoUNet(**kw).eval()
@@ -67,7 +68,13 @@ def _unet_case(ns, tag: str, model_channels: int, T: int, hw: int, wseed: int, s
     err = _pin(tag, ref, ora)
     for w in want:
         _pin(f"{tag}:{w}", taps_ref[w], taps_or[w])
-    blob = {"out": ref, "timesteps": ts}
+    if full_items is None:
+        blob = {"out": ref, "timesteps": ts}
+    else:
+        # BASELINE-size fixture (files stay below 1 MB): `full_items` complete batch items + every stride-th pixel of all
+        # items, fp16 (rounding 5e-4 relative, far below the tolerance); an odd stride samples every pixel parity
+        blob = {"timesteps": ts, "full_items": list(full_items), "out_full": ref[list(full_items)].half(),
+                "stride": stride, "out_sub": ref[:, :, ::stride, ::stride].half()}
     for w in want:
         # keep fixtures small: frames {0 (uc half), T (c half)}, every 8th channel, fp16
         # (tap_stride > 1: also every tap_stride-th pixel -- the BASELINE-size fixture)
@@ -75,7 +82,8 @@ def _unet_case(ns, tag: str, model_channels: int, T: int, hw: int, wseed: int, s
     torch.save(blob, OUT / f"{tag}.pt")
     manifest[tag] = dict(kind="unet_forward", model_channels=model_channels, T=T, latent_hw=hw, weight_seed=wseed,
                          input_seed=23, sigma=sigma, pin_err=err, ref_cpu_seconds=round(t_ref, 2),
-                         out_std=ref.std().item(), tap_stride=tap_stride)
+                         out_std=ref.std().item(), tap_stride=tap_stride,
+                         full_items=list(full_items) if full_items is not None else None, stride=stride)
     return net, sd, spec
 
 
@@ -138,7 +146,7 @@ def _sampler_variant_case(ns, net, sd, spec, tag: str, T: int, hw: int, num_step
 
 
 def _decoder_case(ns, tag: str, ch: int, T: int, B: int, hw: int, wseed: int, manifest: dict, z=None,
-                  full_frames=None, stride: int = 1):
+                  full_frames=None, stride: int = 1, crop: int = 0):
     kw = dict(reference_shim.V3D_DECODER_KW)
     kw["ch"] = ch
     dec = ns.temporal_ae.VideoDecoder(**kw).eval()
@@ -148,8 +156,7 @@ def _decoder_case(ns, tag: str, ch: int, T: int, B: int, hw: int, wseed: int, ma
     sd = synth.synth_state_dict(shapes, seed=wseed)
     dec.load_state_dict(sd)
     if z is None:
-        g = torch.Generator().manual_seed(77)
-        z = torch.randn(B, 4, hw, hw, generator=g)
+        z = synth.synth_latents(B, hw, seed=77)
     with torch.no_grad():
         t0 = time.time()
         # decode_first_stage semantics (video_diffusion.py:182-210): z / scale_factor, one chunk of T frames
@@ -161,13 +168,17 @@ def _decoder_case(ns, tag: str, ch: int, T: int, B: int, hw: int, wseed: int, ma
     if full_frames is None:
         torch.save({"out": ref, "z": z}, OUT / f"{tag}.pt")
     else:
-        # BASELINE-size fixture: `full_frames` complete frames + every stride-th pixel of all frames, fp16
-        # (the decoder output is an image in about [-1.5, 1.5]: fp16 rounding 5e-4 relative, far below the tolerance)
-        torch.save({"z": z, "full_frames": list(full_frames), "out_full": ref[list(full_frames)].half(),
+        # BASELINE-size fixture (files stay below 1 MB): the top-left crop x crop pixels of the `full_frames` at full
+        # resolution + every stride-th pixel of all frames, fp16 (the decoder output is an image in about [-1.5, 1.5]:
+        # fp16 rounding 5e-4 relative, far below the tolerance).  z is regenerated from its seed
+        # (synth.synth_latents); z_check, every 16th latent pixel, pins that
+        torch.save({"z_check": z[:, :, ::16, ::16].clone(), "full_frames": list(full_frames),
+                    "out_full": ref[list(full_frames), :, :crop, :crop].half(), "crop": crop,
                     "stride": stride, "out_sub": ref[:, :, ::stride, ::stride].half()}, OUT / f"{tag}.pt")
     manifest[tag] = dict(kind="decode", ch=ch, T=T, B=B, latent_hw=hw, weight_seed=wseed, z_seed=77, pin_err=err,
                          ref_cpu_seconds=round(t_ref, 2), out_std=ref.std().item(),
-                         full_frames=list(full_frames) if full_frames is not None else None, stride=stride)
+                         full_frames=list(full_frames) if full_frames is not None else None, stride=stride,
+                         crop=crop or None)
 
 
 def _encoder_case(ns, tag: str, ch: int, B: int, hw: int, wseed: int, manifest: dict):
@@ -263,6 +274,29 @@ def _conditioning_case(ns, tag: str, T: int, hw: int, manifest: dict):
     manifest[tag] = dict(kind="conditioning", T=T, latent_hw=hw, fps_id=fps_id, motion_bucket_id=motion, cond_aug=aug)
 
 
+def _engine_state_dict_case(tag: str, manifest: dict):
+    """The reference's DiffusionEngine (video_diffusion.py:35-105) built from the small V3D_512 config with its own
+    `target:`s: the name, shape and dtype of every state_dict entry (what a checkpoint of the reference carries).  The
+    same engine class built from the drop-in targets must produce the same table."""
+    reference_shim._stub("kornia")
+    reference_shim._stub("open_clip")
+    mods = sys.modules["sgm.modules"]
+    enc = importlib.import_module("sgm.modules.encoders.modules")
+    # what sgm/modules/__init__.py:1-6 defines (the package __init__ itself is bypassed by the shim: it pulls CLIP)
+    mods.GeneralConditioner = enc.GeneralConditioner
+    mods.UNCONDITIONAL_CONFIG = {"target": "sgm.modules.GeneralConditioner", "params": {"emb_models": []}}
+    engine_cls = importlib.import_module("sgm.models.video_diffusion").DiffusionEngine
+    table = lambda sd: [[k, list(v.shape), str(v.dtype).replace("torch.", "")] for k, v in sd.items()]  # noqa: E731
+    ref = table(engine_cls(**reference_shim.engine_config_small("sgm")).state_dict())
+    drop = table(engine_cls(**reference_shim.engine_config_small("v3d_b200.sgm")).state_dict())
+    if sorted(ref) != sorted(drop):
+        raise SystemExit(f"{tag}: the reference engine builds different state_dicts from the drop-in targets")
+    with gzip.GzipFile(OUT / f"{tag}.json.gz", "wb", mtime=0) as f:
+        f.write(json.dumps({"state_dict": ref}).encode())
+    manifest[tag] = dict(kind="engine_state_dict", entries=len(ref), config="oracle.reference_shim.engine_config_small")
+    print(f"  {tag}: {len(ref)} state_dict entries, drop-in targets identical")
+
+
 def main(argv):
     OUT.mkdir(parents=True, exist_ok=True)
     ns = reference_shim.load()
@@ -292,7 +326,8 @@ def main(argv):
         _edm_step_case(ns, net, sd, spec, "edm_full_step", T=4, hw=32, num_steps=1, manifest=manifest)
     if want("unet_v3d512"):
         # BASELINE.json configs[1] network evaluation: full width, T=18, latent 64x64, CFG batch 36 (one forward)
-        _unet_case(ns, "unet_v3d512", 320, T=18, hw=64, wseed=3, sigma=3.0, manifest=manifest, tap_stride=4)
+        _unet_case(ns, "unet_v3d512", 320, T=18, hw=64, wseed=3, sigma=3.0, manifest=manifest, tap_stride=4,
+                   full_items=(0, 18 + 11), stride=3)
     if want("edm_v3d512_25step"):
         # 25 accumulating Euler-EDM steps (CFG, T=18) on the full-width network at the smallest latent that
         # exercises every level (16x16 -> 2x2 at the bottom)
@@ -301,7 +336,7 @@ def main(argv):
     if want("decoder_v3d512"):
         # BASELINE.json configs[1] decode: 18 frames, latent 64x64 -> 512x512, one chunk
         _decoder_case(ns, "decoder_v3d512", 128, T=18, B=18, hw=64, wseed=6, manifest=manifest,
-                      full_frames=(0, 11), stride=4)
+                      full_frames=(0, 11), stride=8, crop=160)
     if want("decoder_small"):
         _decoder_case(ns, "decoder_small", 64, T=3, B=3, hw=16, wseed=4, manifest=manifest)
     if want("decoder_small_2videos"):
@@ -319,6 +354,8 @@ def main(argv):
         _clip_case("clip_vit_h14", ref_clip.ClipSpec(), B=1, img_hw=512, wseed=22, manifest=manifest)
     if want("conditioning"):
         _conditioning_case(ns, "conditioning", T=18, hw=8, manifest=manifest)
+    if want("engine_state_dict_small"):
+        _engine_state_dict_case("engine_state_dict_small", manifest)
     # integer / index paths: sigma schedule and guider scale, bit-exact
     if want("schedule"):
         disc = ns.discretizer.EDMDiscretization(sigma_max=700.0)

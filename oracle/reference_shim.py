@@ -7,6 +7,7 @@ placeholders (SURVEY.md §8(c)).  /root/reference does not exist on the GPU box;
 """
 from __future__ import annotations
 
+import copy
 import importlib
 import sys
 import types
@@ -101,3 +102,30 @@ V3D_DECODER_KW = dict(  # scripts/pub/configs/V3D_512.yaml:111-132
     attn_type="vanilla", double_z=True, z_channels=4, resolution=256, in_channels=3, out_ch=3, ch=128,
     ch_mult=[1, 2, 4, 4], num_res_blocks=2, attn_resolutions=[], dropout=0.0, video_kernel_size=[3, 1, 1],
 )
+
+
+def engine_config_small(prefix: str, width: int = 64, dec_ch: int = 64, T: int = 4) -> dict:
+    """scripts/pub/configs/V3D_512.yaml:17-146 with the `target:` prefix of the path components as a parameter
+    ("sgm": the reference's classes, "v3d_b200.sgm": the drop-ins) and reduced widths (construction cost only)."""
+    dm = prefix + ".modules.diffusionmodules."
+    return copy.deepcopy(dict(
+        scale_factor=0.18215, disable_first_stage_autocast=True, input_key="latents", log_keys=[], en_and_decode_n_samples_a_time=T,
+        denoiser_config={"target": dm + "denoiser.Denoiser",
+                         "params": {"scaling_config": {"target": dm + "denoiser_scaling.VScalingWithEDMcNoise"}}},
+        network_config={"target": dm + "video_model.VideoUNet",
+                        "params": dict(V3D_UNET_KW, model_channels=width)},
+        first_stage_config={
+            "target": prefix + ".models.autoencoder.AutoencodingEngine",
+            "params": {
+                "loss_config": {"target": "torch.nn.Identity"},
+                "regularizer_config": {"target": prefix + ".modules.autoencoding.regularizers.DiagonalGaussianRegularizer"},
+                "encoder_config": {"target": "torch.nn.Identity"},
+                "decoder_config": {"target": prefix + ".modules.autoencoding.temporal_ae.VideoDecoder",
+                                   "params": dict(V3D_DECODER_KW, ch=dec_ch)}}},
+        sampler_config={"target": dm + "sampling.EulerEDMSampler",
+                        "params": {"num_steps": 3,
+                                   "discretization_config": {"target": dm + "discretizer.EDMDiscretization",
+                                                             "params": {"sigma_max": 700.0}},
+                                   "guider_config": {"target": dm + "guiders.LinearPredictionGuider",
+                                                     "params": {"max_scale": 3.5, "min_scale": 3.5, "num_frames": T}}}},
+    ))

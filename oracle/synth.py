@@ -56,3 +56,10 @@ def synth_inputs(T: int, latent_hw: int, seed: int = 23, ctx_dim: int = 1024, ad
     c = {"crossattn": cross, "concat": concat, "vector": vector}
     uc = {"crossattn": torch.zeros_like(cross), "concat": torch.zeros_like(concat), "vector": vector.clone()}
     return x, c, uc
+
+
+def synth_latents(B: int, latent_hw: int, seed: int = 77) -> torch.Tensor:
+    """Latents [B, 4, h, w] ~ N(0, 1) for the decode fixtures."""
+    g = torch.Generator(device="cpu")
+    g.manual_seed(seed)
+    return torch.randn(B, 4, latent_hw, latent_hw, generator=g)

@@ -368,6 +368,32 @@ def test_bench_native_line_assembly():
     assert one["e2e"]["d2h_bytes_per_step"] == 14155776 and "plan 'cfg'" in one["config"]["parallelism"]
 
 
+def test_bench_dump_outputs_complete_or_seeded_sample(tmp_path):
+    """bench.py --dump-outputs: arrays within the byte budget are written whole as float32; over it, every array
+    becomes the same fixed sample from run to run, and the files stay within the budget."""
+    import numpy as np
+
+    import bench
+
+    frames = np.random.default_rng(1).integers(0, 256, (3, 16, 16, 3), dtype=np.uint8)
+    info = bench.dump_outputs(tmp_path / "whole", {"frames": frames})
+    got = np.load(tmp_path / "whole" / "frames.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, frames.astype(np.float32))
+    assert info == {"frames": {"shape": [3, 16, 16, 3], "dtype": "float32", "sampled_elements": None}}
+
+    big = {"a": np.arange(40000, dtype=np.float64), "b": np.linspace(0, 1, 10000)}
+    limit = 20000 * 4 + 256
+    runs = [bench.dump_outputs(tmp_path / str(i), big, limit_bytes=limit) for i in range(2)]
+    assert runs[0] == runs[1] and runs[0]["a"]["sampled_elements"] == 16000 and runs[0]["b"]["shape"] == [10000]
+    size = 0
+    for name, full in big.items():
+        one, two = (np.load(tmp_path / str(i) / f"{name}.npy") for i in range(2))
+        assert one.dtype == np.float32 and np.array_equal(one, two)
+        assert np.isin(one, full.astype(np.float32)).all() and np.all(np.diff(one) > 0)   # sorted indices, no repeats
+        size += (tmp_path / "0" / f"{name}.npy").stat().st_size
+    assert size <= limit
+
+
 def test_schedule_cost_accounting_matches_known_flop_budget():
     """tools/schedule_cost.py (meta-device dry run of the launch schedules): the algorithmic FLOPs it books for the
     V3D_512 UNet forward and decode agree with the reference accounting of SURVEY.md App. B minus the documented

@@ -1,21 +1,22 @@
-"""Boundary proof with the REFERENCE's own plugin machinery (SURVEY.md 8(b); VERDICT r1 item 9).
+"""Checkpoint compatibility with the reference's DiffusionEngine (SURVEY.md 8(b); INTEGRATION.md section A).
 
-The reference's `DiffusionEngine.__init__` (sgm/models/video_diffusion.py:35-105) is run - unmodified, imported in place
-from /root/reference through oracle/reference_shim.py - on a config whose hot-path `target:` strings are the drop-ins of
-INTEGRATION.md section A.  `instantiate_from_config` / `get_obj_from_str` (sgm/util.py:170-187) therefore resolve and
-construct the v3d_b200 classes exactly as `scripts/pub/V3D_512.py:72-112` would.  Checked:
+tests/golden/engine_state_dict_small.json.gz holds the name, shape and dtype of every `state_dict()` entry of the
+reference's `DiffusionEngine` (sgm/models/video_diffusion.py:35-105) built from the small V3D_512 config of
+`oracle.reference_shim.engine_config_small` with the reference's own `target:`s (oracle/make_golden.py, which also
+checks that the reference engine class builds the same table from the drop-in targets).  Checked here, on the drop-in
+`v3d_b200.sgm.models.video_diffusion.DiffusionEngine` built from the drop-in `target:`s of INTEGRATION.md section A:
 
-  * the engine the reference builds from the drop-in targets has the SAME `state_dict()` keys and shapes as the engine it
-    builds from its own targets (network, first-stage decoder; the conditioner is the reference's unconditional stub);
-  * `load_state_dict(strict=True)` of the reference-built engine's weights into the drop-in-built engine;
-  * the reference's `init_from_ckpt` (video_diffusion.py:123-168, safetensors branch) loads a checkpoint written from the
-    reference-built engine into the drop-in-built engine with no missing / unexpected keys;
-  * the drop-in `v3d_b200.sgm.models.video_diffusion.DiffusionEngine` accepts the same checkpoint.
+  * `instantiate_from_config` resolves the drop-in targets to the v3d_b200 classes;
+  * its `state_dict()` has the SAME names, shapes and dtypes as the reference engine's (network, first-stage decoder,
+    and nothing else: the conditioner is the unconditional stub, the denoiser / sampler hold no parameters);
+  * `load_state_dict(strict=True)` of a state dict with the reference's layout, and back;
+  * `init_from_ckpt` (the safetensors branch of video_diffusion.py:123-168) loads a checkpoint with the reference's
+    layout with no missing / unexpected keys.
 
-CPU only (construction and weight plumbing; no kernels run).  Skipped where /root/reference is absent (the GPU box).
+CPU only (construction and weight plumbing; no kernels run).
 """
-import copy
-import importlib
+import gzip
+import json
 import sys
 from pathlib import Path
 
@@ -27,97 +28,56 @@ sys.path.insert(0, str(ROOT))
 
 from oracle import reference_shim  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not reference_shim.available(), reason="/root/reference not present")
-
-WIDTH, DEC_CH, T = 64, 64, 4
-
-
-def _config(prefix: str, first_stage_prefix: str):
-    """scripts/pub/configs/V3D_512.yaml:17-146 with the `target:` prefix of the hot-path components as a parameter
-    (reduced widths: construction cost only)."""
-    dm = prefix + ".modules.diffusionmodules."
-    return dict(
-        scale_factor=0.18215, disable_first_stage_autocast=True, input_key="latents", log_keys=[], en_and_decode_n_samples_a_time=T,
-        denoiser_config={"target": dm + "denoiser.Denoiser",
-                         "params": {"scaling_config": {"target": dm + "denoiser_scaling.VScalingWithEDMcNoise"}}},
-        network_config={"target": dm + "video_model.VideoUNet",
-                        "params": dict(adm_in_channels=768, num_classes="sequential", use_checkpoint=False, in_channels=8,
-                                       out_channels=4, model_channels=WIDTH, attention_resolutions=[4, 2, 1],
-                                       num_res_blocks=2, channel_mult=[1, 2, 4, 4], num_head_channels=64,
-                                       use_linear_in_transformer=True, transformer_depth=1, context_dim=1024,
-                                       spatial_transformer_attn_type="softmax", extra_ff_mix_layer=True,
-                                       use_spatial_context=True, merge_strategy="learned_with_images",
-                                       video_kernel_size=[3, 1, 1])},
-        first_stage_config={
-            "target": first_stage_prefix + ".models.autoencoder.AutoencodingEngine",
-            "params": {
-                "loss_config": {"target": "torch.nn.Identity"},
-                "regularizer_config": {"target": "sgm.modules.autoencoding.regularizers.DiagonalGaussianRegularizer"},
-                "encoder_config": {"target": "torch.nn.Identity"},
-                "decoder_config": {"target": prefix + ".modules.autoencoding.temporal_ae.VideoDecoder",
-                                   "params": dict(attn_type="vanilla", double_z=True, z_channels=4, resolution=256,
-                                                  in_channels=3, out_ch=3, ch=DEC_CH, ch_mult=[1, 2, 4, 4],
-                                                  num_res_blocks=2, attn_resolutions=[], dropout=0.0,
-                                                  video_kernel_size=[3, 1, 1])}}},
-        sampler_config={"target": dm + "sampling.EulerEDMSampler",
-                        "params": {"num_steps": 3,
-                                   "discretization_config": {"target": dm + "discretizer.EDMDiscretization",
-                                                             "params": {"sigma_max": 700.0}},
-                                   "guider_config": {"target": dm + "guiders.LinearPredictionGuider",
-                                                     "params": {"max_scale": 3.5, "min_scale": 3.5, "num_frames": T}}}},
-    )
+GOLD = ROOT / "tests" / "golden" / "engine_state_dict_small.json.gz"
 
 
 @pytest.fixture(scope="module")
-def ref_engine_cls():
-    reference_shim.install()
-    reference_shim._stub("kornia")
-    reference_shim._stub("open_clip")
-    mods = sys.modules["sgm.modules"]
-    enc = importlib.import_module("sgm.modules.encoders.modules")
-    # what sgm/modules/__init__.py:1-6 defines (the package __init__ itself is bypassed by the shim: it pulls CLIP)
-    mods.GeneralConditioner = enc.GeneralConditioner
-    mods.UNCONDITIONAL_CONFIG = {"target": "sgm.modules.GeneralConditioner", "params": {"emb_models": []}}
-    vd = importlib.import_module("sgm.models.video_diffusion")
-    return vd.DiffusionEngine
+def ref_table():
+    with gzip.open(GOLD, "rt") as f:
+        return {k: (tuple(shape), getattr(torch, dtype)) for k, shape, dtype in json.load(f)["state_dict"]}
 
 
 @pytest.fixture(scope="module")
-def engines(ref_engine_cls):
+def drop():
+    from v3d_b200.sgm.models.video_diffusion import DiffusionEngine
+
     torch.manual_seed(0)
-    ref = ref_engine_cls(**copy.deepcopy(_config("sgm", "sgm")))
-    drop = ref_engine_cls(**copy.deepcopy(_config("v3d_b200.sgm", "v3d_b200.sgm")))
-    return ref, drop
+    return DiffusionEngine(**reference_shim.engine_config_small("v3d_b200.sgm"))
 
 
-def _hot_path_items(sd):
-    return {k: tuple(v.shape) for k, v in sd.items()
+def _ref_state_dict(ref_table):
+    """A state dict with the reference engine's layout and seeded values."""
+    g = torch.Generator().manual_seed(0)
+    return {k: torch.randn(shape, generator=g).to(dtype) for k, (shape, dtype) in ref_table.items()}
+
+
+def _hot_path_items(table):
+    return {k: v for k, v in table.items()
             if k.startswith("model.diffusion_model.") or k.startswith("first_stage_model.decoder.")}
 
 
-def test_reference_loader_builds_dropins_with_identical_state_dict(engines):
-    ref, drop = engines
+def test_reference_loader_builds_dropins_with_identical_state_dict(drop, ref_table):
     import v3d_b200.decoder
     import v3d_b200.sampling
     import v3d_b200.unet
 
-    # the reference's instantiate_from_config constructed OUR classes
+    # instantiate_from_config constructed OUR classes
     assert isinstance(drop.model.diffusion_model, v3d_b200.unet.VideoUNet)
     assert isinstance(drop.first_stage_model.decoder, v3d_b200.decoder.VideoDecoder)
     assert isinstance(drop.sampler, v3d_b200.sampling.EulerEDMSampler)
     assert isinstance(drop.denoiser, v3d_b200.sampling.Denoiser)
-    assert type(drop.model).__module__ == "sgm.modules.diffusionmodules.wrappers"     # the reference's own wrapper
-    a, b = _hot_path_items(ref.state_dict()), _hot_path_items(drop.state_dict())
+    assert isinstance(drop.model, v3d_b200.sampling.OpenAIWrapper)
+    mine = {k: (tuple(v.shape), v.dtype) for k, v in drop.state_dict().items()}
+    a, b = _hot_path_items(ref_table), _hot_path_items(mine)
     assert len(a) > 1000 and a == b
-    # nothing else differs either (conditioner stub has no weights; the denoiser / sampler hold no parameters)
-    extra_ref = set(ref.state_dict()) - set(a)
-    extra_drop = set(drop.state_dict()) - set(b)
+    # nothing else differs either
+    extra_ref = set(ref_table) - set(a)
+    extra_drop = set(mine) - set(b)
     assert extra_ref == extra_drop, (sorted(extra_ref ^ extra_drop)[:10])
 
 
-def test_strict_load_state_dict_round_trip(engines):
-    ref, drop = engines
-    sd = {k: v.clone() for k, v in ref.state_dict().items()}
+def test_strict_load_state_dict_round_trip(drop, ref_table):
+    sd = _ref_state_dict(ref_table)
     missing, unexpected = drop.load_state_dict(sd, strict=True)
     assert not missing and not unexpected
     back = drop.state_dict()
@@ -126,23 +86,16 @@ def test_strict_load_state_dict_round_trip(engines):
         assert torch.equal(back[k], sd[k]), k
 
 
-def test_reference_init_from_ckpt_loads_into_dropins(engines, ref_engine_cls, tmp_path):
+def test_reference_init_from_ckpt_loads_into_dropins(ref_table, tmp_path):
     from safetensors.torch import save_file
 
-    ref, drop = engines
-    path = str(tmp_path / "v3d_small.safetensors")
-    save_file({k: v.contiguous() for k, v in ref.state_dict().items()}, path)
-    # 1) the REFERENCE engine class, drop-in targets, the reference's own checkpoint loader
-    cfg = copy.deepcopy(_config("v3d_b200.sgm", "v3d_b200.sgm"))
-    eng = ref_engine_cls(ckpt_path=path, **cfg)
-    want = ref.state_dict()
-    got = eng.state_dict()
-    for k, v in want.items():
-        assert torch.equal(got[k], v), k
-    # 2) the drop-in engine class on the same checkpoint and config
     from v3d_b200.sgm.models.video_diffusion import DiffusionEngine
 
-    eng2 = DiffusionEngine(ckpt_path=path, **copy.deepcopy(cfg))
-    got2 = eng2.state_dict()
-    for k in _hot_path_items(want):
-        assert torch.equal(got2[k], want[k]), k
+    want = _ref_state_dict(ref_table)
+    path = str(tmp_path / "v3d_small.safetensors")
+    save_file(want, path)
+    eng = DiffusionEngine(ckpt_path=path, **reference_shim.engine_config_small("v3d_b200.sgm"))
+    got = eng.state_dict()
+    assert set(got) == set(want)
+    for k, v in want.items():
+        assert torch.equal(got[k], v), k
